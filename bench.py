@@ -4,6 +4,7 @@ audio samples/sec (22.05 kHz) at N=4 reverse steps).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # CPU yardstick (oracle port of the reference)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's output as DIR/<name>.npy
 
 A "step" = one complete sampling call (all N=4 reverse steps incl. noise generation) over one batch of
 synthetic input.  Workload at every N: BASELINE.json configs[1] per GPU -- batch 8 x 10 s synthetic mel
@@ -26,6 +27,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 N4_SCHEDULE = [3.2176e-04, 2.5743e-03, 2.5376e-02, 7.0414e-01]  # modules/FastDiff/task/FastDiff.py:88-89
@@ -164,8 +166,8 @@ class CpuYardstick:
     """The reference's CPU implementation of the path on the host cores (fp32, all intra-op threads).
 
     kind "reference": the UNMODIFIED reference (`sampling_given_noise_schedule` over `FastDiff.forward`,
-    modules/FastDiff/module/util.py:158-235) imported from /root/reference or from the staged copy baseline/_ref
-    (oracle/stage_reference.py), `.cuda()` shimmed to identity.  kind "port": oracle/fastdiff_oracle.py -- only when no copy of
+    modules/FastDiff/module/util.py:158-235) imported from the checkout named by FD_REFERENCE_ROOT or from its bytecode build
+    oracle/_ref (oracle/stage_reference.py), `.cuda()` shimmed to identity.  kind "port": oracle/fastdiff_oracle.py -- only when no copy of
     the reference is reachable (it is ~3.8x slower than the reference: its LVC is three einsum taps where the reference unfolds
     once and calls bmm; say so wherever the number is shown)."""
 
@@ -305,12 +307,13 @@ def run_ours(args):
         clocks.mark_begin()
     ev0.record()
     for i in range(args.steps):
-        one_call(args.warmup + i)
+        out = one_call(args.warmup + i)
     ev1.record()
     barrier()
     if clocks:
         clocks.mark_end()
     ms = ev0.elapsed_time(ev1)
+    last_out = out.cpu() if args.dump_outputs else None
     launches = eng.launch_count() - l0
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -414,6 +417,8 @@ def run_ours(args):
             log("e2e (reference noise) leg failed:", repr(e))
 
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"audio" if world == 1 else f"audio_rank{rank}": last_out}, DUMP_LIMIT_BYTES // world)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -511,6 +516,22 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays, limit):
+    """Write each array as float32 `path/<name>.npy`.  An array over `limit` bytes (with --batch / --frames far above the default) is
+    replaced by the fixed sample flat[::stride] with the smallest stride that fits, so two builds still compare element for element."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.to(torch.float32).numpy()
+        stride = -(-a.nbytes // limit)
+        if stride > 1:
+            a = a.reshape(-1)[::stride]
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        log(f"dump: {name} {a.shape} -> {path}" + (f" (flat[::{stride}])" if stride > 1 else ""))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -522,7 +543,11 @@ def main():
     ap.add_argument("--frames", type=int, default=861)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--opt", action="append", default=[], help="library tuning option key=value (fd_set_option), repeatable")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the waveform the last timed step returned as DIR/audio.npy (float32, at most 64 MB; one file per rank)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -21,11 +21,10 @@ Reference files restated (all under /root/reference):
 
 Pinning: the reference ships no tests or golden vectors for this path
 (SURVEY.md section 4), so the oracle is pinned against the reference itself:
-  * tests/test_oracle_vs_reference.py imports the reference from
-    /root/reference (when present -- i.e. in the build container) and checks
-    every function here against it on seeded inputs;
   * tests/golden/*.npz are outputs of the imported reference, produced by
-    tests/golden/make_golden.py (committed), and are checked on any box.
+    tests/golden/make_golden.py (committed), and are checked on any machine;
+  * tests/test_oracle_vs_reference.py checks every function here against
+    the reference's outputs for the same seeded inputs (reference_cpu.npz).
 """
 from __future__ import annotations
 

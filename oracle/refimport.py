@@ -1,7 +1,8 @@
 """Import the UNMODIFIED reference (test / benchmark infrastructure only -- never imported by ``fastdiff_b200/``).
 
-``reference_root()`` = ``/root/reference`` in the build container, else the staged copy ``baseline/_ref`` (oracle/stage_reference.py),
-else None.  ``load(device)`` puts it on ``sys.path`` and returns the hot-path symbols.  The reference hard-codes ``.cuda()``
+``reference_root()`` = the checkout named by ``FD_REFERENCE_ROOT``, else the bytecode build ``oracle/_ref`` (oracle/stage_reference.py),
+else None; ``reference_checkout()`` = a source checkout with the YAML configs: ``FD_REFERENCE_ROOT``, else the one ``oracle/_ref`` was
+built from, if it is still reachable.  ``load(device)`` puts it on ``sys.path`` and returns the hot-path symbols.  The reference hard-codes ``.cuda()``
 (util.py:68,91,217,427); for a CPU run ``torch.Tensor.cuda`` is shimmed to identity (SURVEY.md 8c) -- nothing else is touched.
 The task-level import chain additionally needs packages that are absent from this image (chardet, librosa, resemblyzer); they are
 stubbed with empty modules -- none of them is used by ``test_step`` / ``spec2wav``.
@@ -16,16 +17,26 @@ import warnings
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-_CANDIDATES = ("/root/reference", os.path.join(ROOT, "baseline", "_ref"))
+BUILT = os.path.join(ROOT, "oracle", "_ref")
 _orig_tensor_cuda = torch.Tensor.cuda
 
 
 def reference_root():
-    forced = os.environ.get("FD_REFERENCE_ROOT")            # tests: force the staged copy even where /root/reference exists
-    for c in ((forced,) if forced else _CANDIDATES):
-        if os.path.isdir(os.path.join(c, "modules", "FastDiff", "module")):
+    for c in (os.environ.get("FD_REFERENCE_ROOT"), BUILT):
+        if c and os.path.isdir(os.path.join(c, "modules", "FastDiff", "module")):
             return c
     return None
+
+
+def reference_checkout():
+    c = os.environ.get("FD_REFERENCE_ROOT")
+    if not c:
+        try:
+            with open(os.path.join(BUILT, "SOURCE")) as fh:
+                c = fh.read().strip()
+        except OSError:
+            return None
+    return c if os.path.isfile(os.path.join(c, "modules", "FastDiff", "config", "FastDiff.yaml")) else None
 
 
 def shim_cuda_to_cpu(on: bool = True):
@@ -64,7 +75,7 @@ def load(device: str = "cpu"):
     """-> namespace(root, FastDiff, sampling_given_noise_schedule, compute_hyperparams_given_schedule, util, modules)."""
     root = reference_root()
     if root is None:
-        raise FileNotFoundError("reference not available: neither /root/reference nor baseline/_ref (run oracle/stage_reference.py)")
+        raise FileNotFoundError("reference not available: set FD_REFERENCE_ROOT to a checkout of it (oracle/stage_reference.py builds oracle/_ref)")
     if root not in sys.path:
         sys.path.insert(0, root)
     shim_cuda_to_cpu(device == "cpu")

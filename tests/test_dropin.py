@@ -6,7 +6,9 @@
   * the vocoder registry (vocoders/base_vocoder.py:3-40): `register_vocoder(FastDiffVocoder)`, `get_vocoder_cls(hparams)` by name and by
     dotted path, `spec2wav(mel [T, 80])` as tasks/tts/tts_base.py:254,284 call it.
 
-The reference is imported from /root/reference (build container) or from the staged copy baseline/_ref (GPU box; oracle/stage_reference.py).
+The reference is imported from the checkout named by FD_REFERENCE_ROOT or from the bytecode build oracle/_ref that __graft_entry__.build()
+makes of a reachable checkout (oracle/stage_reference.py); the task test reads the reference's YAML configs, so it needs the checkout.
+Where neither is reachable (a GPU machine without the reference), these tests skip.
 CPU variant: through the emulation build of the CUDA source; `-m gpu` variant: the real library on cuda:0."""
 import os
 import sys
@@ -19,11 +21,11 @@ import torch
 N4 = [3.2176e-04, 2.5743e-03, 2.5376e-02, 7.0414e-01]
 
 
-def _reference(device, monkeypatch):
+def _reference(device, monkeypatch, configs=False):
     from oracle import refimport
-    root = refimport.reference_root()
+    root = refimport.reference_checkout() if configs else refimport.reference_root()
     if root is None:
-        pytest.skip("no copy of the reference reachable (neither /root/reference nor baseline/_ref)")
+        pytest.skip("needs the reference's own code" + (" and YAML configs" if configs else "") + ": no checkout of it is reachable")
     refimport.stub_missing_deps()
     if device == "cpu":
         monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self)
@@ -38,7 +40,7 @@ def _reference(device, monkeypatch):
 
 def _run_task(tmp_path, device, lib_path, synth, monkeypatch):
     import warnings
-    _reference(device, monkeypatch)
+    _reference(device, monkeypatch, configs=True)
     from fastdiff_b200.synthetic import make_inputs
     from oracle import fastdiff_oracle as O
     mel_dir = tmp_path / "mels"

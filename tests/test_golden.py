@@ -22,7 +22,8 @@ def test_oracle_vs_golden_denoise(synth):
     assert (eps - g["eps"]).abs().max() < 2e-5
     for n in range(3):
         assert (inter[f"down{n}"] - g[f"down{n}"]).abs().max() < 1e-5
-        assert (inter[f"lvc{n}"] - g[f"lvc{n}"]).abs().max() < 5e-5
+        lvc, want = (inter[f"lvc{n}"], g[f"lvc{n}"]) if n < 2 else (inter["lvc2"][:, :, ::4], g["lvc2_sub"])
+        assert (lvc - want).abs().max() < 5e-5
 
 
 def test_oracle_vs_golden_sampler(synth):
@@ -77,7 +78,7 @@ def test_emulated_cuda_source_vs_golden_denoise(synth, emu_lib):
         k = eng.debug_read(f"kernels{n}", 2, 12).reshape(2, 4, 32, 64, 3, 12)[:, :, ::8, ::8]
         assert (k - g[f"kernels{n}_sub"]).abs().max() < 2e-5
         assert (eng.debug_read(f"kbias{n}", 2, 12).reshape(2, 4, 64, 12) - g[f"kbias{n}"]).abs().max() < 2e-5
-    assert (eng.debug_read("lvc2", 2, 12).reshape(2, 32, 3072) - g["lvc2"]).abs().max() < 1e-4
+    assert (eng.debug_read("lvc2", 2, 12).reshape(2, 32, 3072)[:, :, ::4] - g["lvc2_sub"]).abs().max() < 1e-4
 
 
 @pytest.mark.gpu
@@ -96,7 +97,7 @@ def test_cuda_vs_golden_denoise(synth, cuda_lib):
         assert (eng.debug_read(f"down{n}", 2, 12).cpu().reshape(2, 32, T) - g[f"down{n}"]).abs().max() < 1e-5
         k = eng.debug_read(f"kernels{n}", 2, 12).cpu().reshape(2, 4, 32, 64, 3, 12)[:, :, ::8, ::8]
         assert (k - g[f"kernels{n}_sub"]).abs().max() < 2e-5
-    assert (eng.debug_read("lvc2", 2, 12).cpu().reshape(2, 32, 3072) - g["lvc2"]).abs().max() < 1e-4
+    assert (eng.debug_read("lvc2", 2, 12).cpu().reshape(2, 32, 3072)[:, :, ::4] - g["lvc2_sub"]).abs().max() < 1e-4
 
 
 @pytest.mark.gpu

@@ -80,8 +80,8 @@ def test_gpu_mel_frontend_matches_oracle(cuda_lib):
 
 
 def test_vocoder_wav2spec_matches_oracle(emu_lib, tmp_path):
-    """`BaseVocoder.wav2spec` shape: (wav, mel [T,80]) from a wav FILE, through the emulated CUDA source; plus the reference's own
-    example audio when the reference tree is mounted (build container only)."""
+    """`BaseVocoder.wav2spec` shape: (wav, mel [T,80]) from a wav FILE, through the emulated CUDA source; a synthetic signal and an
+    excerpt of the reference's own example recording (egs/audios/LJ001-0001_gt.wav, stored under tests/golden)."""
     import os
     from scipy.io import wavfile
     from fastdiff_b200.engine import Engine
@@ -91,10 +91,7 @@ def test_vocoder_wav2spec_matches_oracle(emu_lib, tmp_path):
     pcm = (np.clip(_signals()[1], -1, 1) * 32767).astype(np.int16)
     fn = tmp_path / "a.wav"
     wavfile.write(fn, 22050, pcm)
-    files = [str(fn)]
-    ref_audio = "/root/reference/egs/audios/LJ001-0001_gt.wav"
-    if os.path.exists(ref_audio) and wavfile.read(ref_audio)[0] == 22050:
-        files.append(ref_audio)
+    files = [str(fn), os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "LJ001-0001_gt_excerpt.wav")]
     for f in files:
         wav, mel = FastDiffVocoder.wav2spec(f, engine=eng)
         sr, data = wavfile.read(f)

@@ -1,4 +1,4 @@
-"""Drop-in check with the UNMODIFIED reference task code (build container only): `tasks/run.py`'s import chain resolves,
+"""Drop-in check with the UNMODIFIED reference task code (oracle/refimport.py: reference_checkout): `tasks/run.py`'s import chain resolves,
 `FastDiffTask.build_model` builds the B200 model from the reference's own YAML hparams, and `test_step` drives our sampler
 (through the CPU-emulated CUDA source, so this runs without a GPU) and writes the wav like the reference does."""
 import os
@@ -9,8 +9,10 @@ import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "modules", "FastDiff")), reason="reference not mounted")
+from oracle import refimport
+
+REF = refimport.reference_checkout()
+pytestmark = pytest.mark.skipif(REF is None, reason="needs the reference's own task code and configs: no checkout of it is reachable")
 
 
 def _stub_missing_deps():
